@@ -9,6 +9,7 @@ matrix is all-reduced).  A step is K1 (+K1b) -> K2 over data resident in HBM.
     python bench.py --gpus 1 --steps 20 --warmup 3
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference        # the reference's CPU path (oracle port) on host cores
+    python bench.py --gpus 1 --steps 20 --warmup 3 --dump-outputs DIR   # also write the last step's outputs to DIR
 
 Prints ONE JSON line on rank 0 (everything else goes to stderr).
 """
@@ -32,6 +33,7 @@ D_PER_GPU = 100_000_000
 L2_REG, KERNEL_GRAD_SCALE, DATASET_SIZE = 0.01, 1.0, 50000.0
 CPU_SAMPLE_D = 10_000_000
 METRIC = "svgd_posterior_update_algorithmic_GBps"
+DUMP_COLUMNS = 1 << 20   # columns of `out` --dump-outputs writes: n x 2^20 fp32 = 40 MB at n = 10, inside its 64 MB cap
 
 
 def log(*a):
@@ -161,7 +163,7 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, args.steps), max(1, args.warmup)   # same steps / warm-up as the GPU arm
+    steps, warmup = args.steps, max(1, args.warmup)   # same steps / warm-up as the GPU arm
     gbs, ms, threads, kind, D = cpu_reference_run(steps, warmup)
     line = {
         "impl": "reference", "metric": METRIC, "value": gbs, "unit": "GB/s", "n_gpus": args.gpus, "steps": steps,
@@ -769,17 +771,54 @@ def strong_scaling(ops, bdist, dist, sc, n, world, rank, dev, in_kernel, steps):
     return res
 
 
+def make_inputs(n, D, rank, dev):
+    """Synthetic, device-resident inputs of the timed step: particles X and gradients G [n, D] of this rank's column
+    slice [rank*D, (rank+1)*D), seeded by the rank, so every run with the same arguments gets the same ones."""
+    g = torch.Generator(device=dev).manual_seed(1000 + rank)
+    X = torch.randn(n, D, device=dev, generator=g)
+    X *= (0.05 * (1 + 0.1 * torch.arange(n, device=dev, dtype=torch.float32))).unsqueeze(1)
+    G = torch.randn(n, D, device=dev, generator=g) * 1e-3
+    return X, G
+
+
+def dump_outputs(path, out, sc, world, rank):
+    """--dump-outputs: what a caller of the timed step holds after its last step, as .npy files in `path`.
+    out.npy: the update direction [n, D] of this rank's columns, float32, at DUMP_COLUMNS // world columns drawn
+    without replacement by a fixed seed and kept in column order (every column when D is smaller); with N > 1 each
+    rank writes out_rank<r>.npy.  pair_dist, kernel_K, kernel_A, bandwidth_info (h, median, d_lo, d_hi) and
+    median_sel: the scratch the step leaves, the same on every rank, written by rank 0 (float64; K and A float32).
+    The inputs are seeded, so two builds run with the same arguments can be compared file for file."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    D = out.shape[1]
+    cols = DUMP_COLUMNS // world
+    if D > cols:
+        idx = np.sort(np.random.default_rng(0).choice(D, cols, replace=False))
+        out = out[:, torch.from_numpy(idx).to(out.device)]
+    np.save(os.path.join(path, "out.npy" if world == 1 else f"out_rank{rank}.npy"), out.cpu().numpy())
+    if rank == 0:
+        for name, t in (("pair_dist", sc.dist), ("kernel_K", sc.K), ("kernel_A", sc.A), ("bandwidth_info", sc.info),
+                        ("median_sel", sc.sel.double())):
+            np.save(os.path.join(path, f"{name}.npy"), t.cpu().numpy())
+
+
 # --------------------------------------------------------------------------------------
 def main():
     global D_PER_GPU
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline workload")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--d-per-gpu", type=int, default=D_PER_GPU, help=argparse.SUPPRESS)
     ap.add_argument("--skip-extras", action="store_true", help="skip e2e / cpu baseline / other paths (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
 
     if args.impl == "reference":
         run_reference_arm(args)
@@ -810,14 +849,10 @@ def main():
     _lib.get()  # fail loudly if libbde_b200.so is missing
     peak_gbs, peak_src = measured_peaks()
     warmup = max(3, args.warmup)
-    steps = max(1, args.steps)
+    steps = args.steps
     n, D = N_PARTICLES, D_PER_GPU
 
-    # ---- synthetic, device-resident inputs: this rank's column slice [rank*D, (rank+1)*D) ----
-    g = torch.Generator(device=dev).manual_seed(1000 + rank)
-    X = torch.randn(n, D, device=dev, generator=g)
-    X *= (0.05 * (1 + 0.1 * torch.arange(n, device=dev, dtype=torch.float32))).unsqueeze(1)
-    G = torch.randn(n, D, device=dev, generator=g) * 1e-3
+    X, G = make_inputs(n, D, rank, dev)
     out = torch.empty_like(X)
     sc = ops.SvgdScratch.allocate(n, dev)
 
@@ -867,6 +902,8 @@ def main():
         dist.barrier()
     torch.cuda.synchronize()
     launches = _lib.launch_count - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, sc, world, rank)
 
     total_ms = t_begin.elapsed_time(t_end)
     k1_ms = sum(e[0].elapsed_time(e[1]) for e in evs) / steps
