@@ -58,7 +58,11 @@ def svgd_bandwidth(dist_sums: torch.Tensor, l2_reg: float, kernel_grad_scale: fl
     """
     d = dist_sums.to(torch.float64)
     n = d.shape[0]
-    d = torch.sqrt(d) ** 2
+    # correctly rounded sqrt, then one correctly rounded multiplication, as the kernel does: torch.sqrt on CPU
+    # float64 tensors can be one ulp off (vectorised: torch.sqrt(11000313.0) != math.sqrt(11000313.0)), which
+    # moves the median by an ulp, and by how much depends on the host's SIMD path
+    r = torch.from_numpy(np.sqrt(d.cpu().numpy()))
+    d = r * r
     flat = d.reshape(-1)
     nn_ = flat.numel()
     order = torch.sort(flat, stable=True).indices
