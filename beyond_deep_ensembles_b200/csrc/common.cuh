@@ -255,7 +255,7 @@ __device__ __forceinline__ double warp_sum(double v) {
 // after every peer has published e+1, i.e. after it finished reading e.
 // ----------------------------------------------------------------------------
 constexpr int kPeerMaxRanks = 16;
-constexpr int kPeerMaxVals = 512;   // >= pair_count(BDE_MAX_PARTICLES) = 496
+constexpr int kPeerMaxVals = 512;   // >= pair_count(32) = 496: the exchange covers n <= 32 (larger sums stay rank-local)
 struct PeerBuf {                    // one per rank, cudaMalloc'ed (IPC-shareable), zero-filled
     unsigned long long epoch;       // exchanges completed on this rank (device-side counter)
     unsigned long long timeouts;    // exchanges abandoned after kPeerTimeoutNs (results poisoned with NaN)

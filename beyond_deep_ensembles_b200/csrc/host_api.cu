@@ -46,6 +46,7 @@ extern "C" int bde_svgd_host_pairdist(const float* X_host, int n, int64_t D, int
     if (!X_host || !dX || !dist || n < 1 || n > BDE_MAX_PARTICLES || D < 1 || ld_host < D || chunk_cols < 4 ||
         (chunk_cols & 3))
         return BDE_ERR_INVALID_ARG;
+    if (n > kGenericMaxParticles) return BDE_ERR_UNSUPPORTED_N;   // the host-staged path stops at 32 particles
     HostPipe* p = nullptr;
     int rc = get_pipe(&p);
     if (rc != BDE_OK) return rc;
@@ -75,6 +76,7 @@ extern "C" int bde_svgd_host_apply(const float* G_host, float* out_host, int n, 
     if (!G_host || !out_host || !dX || !dG || !dOut || !dist || !K || !A || n < 1 || n > BDE_MAX_PARTICLES || D < 1 ||
         ld_host < D || chunk_cols < 4 || (chunk_cols & 3) || !(dataset_size > 0.0))
         return BDE_ERR_INVALID_ARG;
+    if (n > kGenericMaxParticles) return BDE_ERR_UNSUPPORTED_N;
     HostPipe* p = nullptr;
     int rc = get_pipe(&p);
     if (rc != BDE_OK) return rc;

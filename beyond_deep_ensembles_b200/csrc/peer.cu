@@ -5,10 +5,32 @@
 // cudaMalloc'ed so that it can be exported with CUDA IPC); every rank maps the buffers of all peers and
 // writes the table of mapped pointers into the header of its reduction workspace.  From then on the last
 // CTA of every grid reduction that uses this workspace completes the sum across ranks inside the launch.
-// The library keeps no state: the caller owns the buffer, the mappings and the workspace.
+// The caller owns the buffer, the mappings and the workspace; the library only remembers which workspaces are
+// attached, so that K1 above 32 particles (more sums than an exchange slot holds) can refuse them.
 #include <cstring>
+#include <mutex>
+#include <set>
 
 #include "common.cuh"
+#include "svgd_internal.h"
+
+namespace bde {
+namespace {
+std::mutex g_attached_mu;
+std::set<const void*> g_attached;   // workspaces attached to a peer set of more than one rank
+void set_attached(const void* ws, bool on) {
+    std::lock_guard<std::mutex> lock(g_attached_mu);
+    if (on)
+        g_attached.insert(ws);
+    else
+        g_attached.erase(ws);
+}
+}  // namespace
+bool peer_attached(const void* ws) {
+    std::lock_guard<std::mutex> lock(g_attached_mu);
+    return g_attached.count(ws) != 0;
+}
+}  // namespace bde
 
 using namespace bde;
 
@@ -75,12 +97,14 @@ extern "C" int bde_peer_attach(void* workspace, size_t workspace_bytes, int worl
     // the ticket (first word) is zero between launches, so the whole header can be rewritten in stream order
     BDE_RETURN_IF_CUDA(cudaMemcpyAsync(workspace, &h, sizeof(h), cudaMemcpyHostToDevice, static_cast<cudaStream_t>(stream)));
     BDE_RETURN_IF_CUDA(cudaStreamSynchronize(static_cast<cudaStream_t>(stream)));  // h lives on this stack frame
+    set_attached(workspace, world > 1);
     return BDE_OK;
 }
 
 extern "C" int bde_peer_detach(void* workspace, size_t workspace_bytes, bde_stream_t stream) {
     if (!workspace || workspace_bytes < kWsHeaderBytes) return BDE_ERR_INVALID_ARG;
     BDE_RETURN_IF_CUDA(cudaMemsetAsync(workspace, 0, sizeof(WsHeader), static_cast<cudaStream_t>(stream)));
+    set_attached(workspace, false);
     return BDE_OK;
 }
 

@@ -44,17 +44,17 @@ svgd_pairdist_scalar_kernel(const float* __restrict__ X, int n, int64_t D, int64
 __global__ void __launch_bounds__(256) svgd_bandwidth_kernel(const double* __restrict__ dist, int n, BandwidthParams bp,
                                                              const void* ws) {
     if (ws && peer_exchange_failed(ws)) return;
-    __shared__ double sd[BDE_MAX_PARTICLES * BDE_MAX_PARTICLES];
-    __shared__ double sk[BDE_MAX_PARTICLES * BDE_MAX_PARTICLES];
-    bandwidth_device<BDE_MAX_PARTICLES * BDE_MAX_PARTICLES>(dist, n, bp, sd, sk);
+    __shared__ double sd[kGenericMaxParticles * kGenericMaxParticles];
+    __shared__ double sk[kGenericMaxParticles * kGenericMaxParticles];
+    bandwidth_device<kGenericMaxParticles * kGenericMaxParticles>(dist, n, bp, sd, sk);
 }
 
 __global__ void __launch_bounds__(256)
 svgd_apply_scalar_kernel(const float* __restrict__ X, const float* __restrict__ G, float* __restrict__ out,
                          const float* __restrict__ K, const float* __restrict__ A, int n, int64_t D, int64_t ldx,
                          int64_t ldg, int64_t ldo) {
-    __shared__ float sK[BDE_MAX_PARTICLES * BDE_MAX_PARTICLES];
-    __shared__ float sA[BDE_MAX_PARTICLES * BDE_MAX_PARTICLES];
+    __shared__ float sK[kGenericMaxParticles * kGenericMaxParticles];
+    __shared__ float sA[kGenericMaxParticles * kGenericMaxParticles];
     griddep_wait();
     for (int e = threadIdx.x; e < n * n; e += blockDim.x) {
         sK[e] = K[e];
@@ -63,7 +63,7 @@ svgd_apply_scalar_kernel(const float* __restrict__ X, const float* __restrict__ 
     __syncthreads();
     for (int64_t c = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; c < D;
          c += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-        float xs[BDE_MAX_PARTICLES], gs[BDE_MAX_PARTICLES];
+        float xs[kGenericMaxParticles], gs[kGenericMaxParticles];
         for (int j = 0; j < n; ++j) {
             xs[j] = __ldg(X + j * ldx + c);
             gs[j] = __ldg(G + j * ldg + c);
@@ -85,8 +85,8 @@ __global__ void __launch_bounds__(256)
 svgd_apply_opt_scalar_kernel(float* X, const float* __restrict__ G, const float* __restrict__ K,
                              const float* __restrict__ A, int n, int64_t D, int64_t ldx, int64_t ldg,
                              const __grid_constant__ BaseOptParams o) {
-    __shared__ float sK[BDE_MAX_PARTICLES * BDE_MAX_PARTICLES];
-    __shared__ float sA[BDE_MAX_PARTICLES * BDE_MAX_PARTICLES];
+    __shared__ float sK[kGenericMaxParticles * kGenericMaxParticles];
+    __shared__ float sA[kGenericMaxParticles * kGenericMaxParticles];
     griddep_wait();
     for (int e = threadIdx.x; e < n * n; e += blockDim.x) {
         sK[e] = K[e];
@@ -96,7 +96,7 @@ svgd_apply_opt_scalar_kernel(float* X, const float* __restrict__ G, const float*
     const bool has_s0 = (OPT == kOptAdam) || (o.momentum != 0.0f && o.buf_initialized);
     for (int64_t c = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; c < D;
          c += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-        float xs[BDE_MAX_PARTICLES], gs[BDE_MAX_PARTICLES];
+        float xs[kGenericMaxParticles], gs[kGenericMaxParticles];
         for (int j = 0; j < n; ++j) {
             xs[j] = X[j * ldx + c];
             gs[j] = __ldg(G + j * ldg + c);
@@ -118,7 +118,7 @@ svgd_apply_opt_scalar_kernel(float* X, const float* __restrict__ G, const float*
 }
 
 // particle counts with a register-resident fast path (explicitly instantiated in svgd_inst_*.cu);
-// any other n <= BDE_MAX_PARTICLES runs the generic runtime-n kernels.
+// any other n <= kGenericMaxParticles runs the generic runtime-n kernels, n up to BDE_MAX_PARTICLES svgd_many.cu.
 #define BDE_FOR_EACH_N(X_) X_(2) X_(3) X_(4) X_(5) X_(6) X_(7) X_(8) X_(9) X_(10) X_(11) X_(12) X_(16) X_(20)
 
 #define X_(N_)                                                                                                     \
@@ -155,6 +155,12 @@ int pairdist_impl(const float* X, int n, int64_t D, int64_t ld, double* dist, in
     size_t need = 0;
     bde_svgd_workspace_bytes(n, &need);
     if (!ws || ws_bytes < need) return BDE_ERR_WORKSPACE;
+    if (n > kGenericMaxParticles) {
+        // the in-kernel exchange carries at most kPeerMaxVals sums: an attached workspace would yield rank-local sums
+        if (peer_attached(ws)) return BDE_ERR_UNSUPPORTED_N;
+        if (!aligned16(X) || ld % 4 != 0) return BDE_ERR_ALIGNMENT;
+        return pairdist_many(X, n, D, ld, dist, accumulate, ws, fuse, bp, st);
+    }
     if (n == 1) {
         if (!accumulate) BDE_RETURN_IF_CUDA(cudaMemsetAsync(dist, 0, sizeof(double), st));
         if (fuse) {
@@ -212,6 +218,7 @@ int apply_impl(const float* X, const float* G, float* out, const float* K, const
     const size_t span_o = sizeof(float) * (static_cast<size_t>(n - 1) * ldo + D);
     if (overlaps(out, span_o, X, span_x) || overlaps(out, span_o, G, span_g)) return BDE_ERR_INVALID_ARG;
     const bool vec_ok = aligned16(X) && aligned16(G) && aligned16(out) && (ldx % 4 == 0) && (ldg % 4 == 0) && (ldo % 4 == 0);
+    if (n > kGenericMaxParticles) return vec_ok ? apply_many(X, G, out, K, A, n, D, ldx, ldg, ldo, st) : BDE_ERR_ALIGNMENT;
     if (!vec_ok || !has_fast_path(n)) {
         int64_t want = (D + 255) / 256;
         const int64_t cap = static_cast<int64_t>(sm_count_cached()) * 4;
@@ -235,6 +242,7 @@ int apply_opt_impl(float* X, const float* G, const float* K, const float* A, int
                    int64_t ldg, const BaseOptParams& o, cudaStream_t st, const NextDistParams* next, size_t ws_bytes) {
     pdl_for_this_apply() = take_chain_hint(st);
     if (!X || !G || !K || !A || n < 1 || n > BDE_MAX_PARTICLES || D < 0 || ldx < D || ldg < D) return BDE_ERR_INVALID_ARG;
+    if (n > kOptMaxParticles) return BDE_ERR_UNSUPPORTED_N;   // no fused base-optimizer form above 32 particles
     if (o.kind != kOptSgd && o.kind != kOptAdam) return BDE_ERR_INVALID_ARG;
     const bool needs_s0 = o.kind == kOptAdam || o.momentum != 0.0f;
     if ((needs_s0 && !o.state0) || (o.kind == kOptAdam && !o.state1)) return BDE_ERR_INVALID_ARG;
@@ -311,7 +319,7 @@ extern "C" int bde_svgd_chain_next(bde_stream_t stream) {
 extern "C" int bde_svgd_workspace_bytes(int n, size_t* bytes) {
     if (!bytes || n < 1 || n > BDE_MAX_PARTICLES) return BDE_ERR_INVALID_ARG;
     const int P = pair_count(n) > 0 ? pair_count(n) : 1;
-    *bytes = grid_reduce_ws_bytes(kMaxCtasPairdist, P);
+    *bytes = grid_reduce_ws_bytes(n > kGenericMaxParticles ? kManyMaxCtas : kMaxCtasPairdist, P);
     return BDE_OK;
 }
 
@@ -336,6 +344,7 @@ extern "C" int bde_svgd_bandwidth(const double* dist, int n, double l2_reg, doub
                                   int32_t* sel, bde_stream_t stream) {
     if (!dist || !K || !A || n < 1 || n > BDE_MAX_PARTICLES || !(dataset_size > 0.0)) return BDE_ERR_INVALID_ARG;
     BandwidthParams bp{l2_reg, kernel_grad_scale, dataset_size, h_override, K, A, info, sel};
+    if (n > kGenericMaxParticles) return bandwidth_many(dist, n, bp, static_cast<cudaStream_t>(stream));
     svgd_bandwidth_kernel<<<1, 256, 0, static_cast<cudaStream_t>(stream)>>>(dist, n, bp, nullptr);
     BDE_CHECK_LAUNCH();
     return BDE_OK;
@@ -413,6 +422,7 @@ extern "C" int bde_svgd_apply_adam(float* X, const float* G, const float* K, con
                                    double beta2, double eps, double weight_decay, int decoupled_weight_decay,
                                    float* out_last, bde_stream_t stream) {
     if (n < 1 || n > BDE_MAX_PARTICLES || step0 < 0) return BDE_ERR_INVALID_ARG;
+    if (n > kOptMaxParticles) return BDE_ERR_UNSUPPORTED_N;
     const BaseOptParams o = adam_params(n, exp_avg, exp_avg_sq, step0, lr, beta1, beta2, eps, weight_decay,
                                         decoupled_weight_decay, out_last);
     return apply_opt_impl(X, G, K, A, n, D, ld, ld, o, static_cast<cudaStream_t>(stream));
@@ -450,6 +460,7 @@ extern "C" int bde_svgd_train_step_adam(float* X, const float* G, const float* K
                                         double h_override, float* K_next, float* A_next, double* info, int32_t* sel,
                                         void* workspace, size_t workspace_bytes, bde_stream_t stream) {
     if (n < 1 || n > BDE_MAX_PARTICLES || step0 < 0) return BDE_ERR_INVALID_ARG;
+    if (n > kOptMaxParticles) return BDE_ERR_UNSUPPORTED_N;
     const BaseOptParams o = adam_params(n, exp_avg, exp_avg_sq, step0, lr, beta1, beta2, eps, weight_decay,
                                         decoupled_weight_decay, out_last);
     const NextDistParams nd = next_params(dist_next, fuse_bandwidth, l2_reg, kernel_grad_scale, dataset_size, h_override,

@@ -46,6 +46,22 @@ struct NextDistParams {
 };
 constexpr int kNextDistMaxParticles = 10;  // all pairs of a column quad in one thread's registers
 
+// Particle counts of the generic runtime-n kernels, the fused base-optimizer forms, the host-staged entries and
+// the in-kernel peer exchange.  n in (kGenericMaxParticles, BDE_MAX_PARTICLES] runs the particle-tiled kernels of
+// svgd_many.cu (K1, K1b, K2 only; 16-byte aligned rows).
+constexpr int kGenericMaxParticles = 32;
+constexpr int kManyMaxCtas = 256;   // grid bound of the particle-tiled K1 (one CTA per SM): sizes its workspace
+
+// peer.cu: is `ws` attached (bde_peer_attach) to a peer set of more than one rank?
+bool peer_attached(const void* ws);
+
+// svgd_many.cu: n in 33..64, X (and G, out) 16-byte aligned with ld % 4 == 0 (checked by the callers)
+int pairdist_many(const float* X, int n, int64_t D, int64_t ld, double* dist, int accumulate, void* ws, int fuse,
+                  const BandwidthParams& bp, cudaStream_t st);
+int bandwidth_many(const double* dist, int n, const BandwidthParams& bp, cudaStream_t st);
+int apply_many(const float* X, const float* G, float* out, const float* K, const float* A, int n, int64_t D,
+               int64_t ldx, int64_t ldg, int64_t ldo, cudaStream_t st);
+
 int pairdist_impl(const float* X, int n, int64_t D, int64_t ld, double* dist, int accumulate, void* ws,
                   size_t ws_bytes, int fuse, const BandwidthParams& bp, cudaStream_t st);
 int apply_impl(const float* X, const float* G, float* out, const float* K, const float* A, int n, int64_t D,

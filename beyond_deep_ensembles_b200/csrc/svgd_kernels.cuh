@@ -284,13 +284,12 @@ __host__ __device__ constexpr int pow2_ceil(int v) {
     return p;
 }
 
-template <int MAXPAD>
-__device__ __forceinline__ void bandwidth_device(const double* dist, int n, const BandwidthParams& bp, double* sd, double* sk) {
+// s_key / s_ord: pow2_ceil(n*n) entries of shared scratch for the sort
+__device__ __forceinline__ void bandwidth_sorted(const double* dist, int n, const BandwidthParams& bp, double* sd,
+                                                 double* sk, double* s_key, int* s_ord) {
     const int tid = threadIdx.x + threadIdx.y * blockDim.x;
     const int nthreads = blockDim.x * blockDim.y;
     const int nn = n * n;
-    __shared__ double s_key[MAXPAD];
-    __shared__ int s_ord[MAXPAD];
     __shared__ double s_sel[2];
     __shared__ int s_idx[2];
     __shared__ double s_h;
@@ -387,6 +386,13 @@ __device__ __forceinline__ void bandwidth_device(const double* dist, int n, cons
         bp.K[e] = static_cast<float>(kij);
         bp.A[e] = static_cast<float>(a);
     }
+}
+
+template <int MAXPAD>
+__device__ __forceinline__ void bandwidth_device(const double* dist, int n, const BandwidthParams& bp, double* sd, double* sk) {
+    __shared__ double s_key[MAXPAD];
+    __shared__ int s_ord[MAXPAD];
+    bandwidth_sorted(dist, n, bp, sd, sk, s_key, s_ord);
 }
 
 

@@ -218,8 +218,10 @@ _PEER_SETS: dict = {}
 def enable_peer_exchange(sc: "ops.SvgdScratch", group=None) -> bool:
     """Attach `sc` to the group's peer set (created on first use).  Collective over the group.  Returns
     False — leaving the NCCL all-reduce form in place — for a single rank, CPU tensors, when
-    BDE_PEER_EXCHANGE=0, or when the ranks cannot map each other's memory (not one node / no P2P)."""
-    if world(group) <= 1 or not sc.ws.is_cuda or os.environ.get("BDE_PEER_EXCHANGE", "1") == "0":
+    BDE_PEER_EXCHANGE=0, when the ranks cannot map each other's memory (not one node / no P2P), or above
+    ops.FUSED_MAX_PARTICLES particles (the in-kernel exchange carries at most 32 * 31 / 2 sums)."""
+    if (world(group) <= 1 or not sc.ws.is_cuda or os.environ.get("BDE_PEER_EXCHANGE", "1") == "0"
+            or sc.n > ops.FUSED_MAX_PARTICLES):
         return False
     if getattr(sc, "peers", None) is not None:
         return True

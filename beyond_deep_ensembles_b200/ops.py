@@ -124,6 +124,8 @@ def svgd_apply(X: torch.Tensor, G: torch.Tensor, out: torch.Tensor, sc: SvgdScra
 
 
 NEXT_KERNEL_MAX_PARTICLES = 10  # single-pass training-step form (kNextDistMaxParticles in csrc/svgd_internal.h)
+MAX_PARTICLES = 64              # BDE_MAX_PARTICLES: K1, K1b and K2 (include/bde_b200.h)
+FUSED_MAX_PARTICLES = 32        # kGenericMaxParticles: fused base-optimizer forms, host-staged entries, peer exchange
 
 
 @dataclass

@@ -24,14 +24,18 @@ def rbf(particles: torch.Tensor, h_override=None):
     (grad_kernel = A X with l2_reg = 0, dataset_size = kernel_grad_scale = 1 and G = 0).
     """
     X = particles.detach().contiguous().float()
-    n = X.shape[0]
+    n, D = X.shape
+    if n > ops.FUSED_MAX_PARTICLES and D % 4:
+        # the kernels for more than 32 particles need rows 16-byte apart: copy into a padded row stride
+        X = torch.zeros(n, (D + 3) // 4 * 4, dtype=X.dtype, device=X.device)[:, :D].copy_(X)
     sc = ops.SvgdScratch.allocate(n, X.device)
     ops.svgd_pairdist(X, sc)
     # out = K*0 + A X with A = c K - c diag(rowsum K), c = 1/h^2  ->  -(grad_kernel)
     ops.svgd_bandwidth(sc, 0.0, 1.0, 1.0, 0.0 if h_override is None else float(h_override))
-    out = torch.empty_like(X)
-    ops.svgd_apply(X, torch.zeros_like(X), out, sc)
-    return sc.K.clone(), -out
+    ld = X.stride(0)
+    out = torch.empty(n, ld, dtype=X.dtype, device=X.device)[:, :D]
+    ops.svgd_apply(X, torch.zeros(n, ld, dtype=X.dtype, device=X.device)[:, :D], out, sc)
+    return sc.K.clone(), -out.contiguous()
 
 
 class SVGDOptimizer(BayesianOptimizer):
@@ -43,10 +47,13 @@ class SVGDOptimizer(BayesianOptimizer):
     works alone like the reference): the torch.distributed group whose ranks each hold a COLUMN SLICE of every
     particle (SURVEY.md §8e); only then are the n x n partial distances summed across ranks.
 
+    `particle_count` is at most ops.MAX_PARTICLES (64); a larger count raises ValueError.
+
     `fuse_base_optimizer` (class attribute, default True): when the base optimizer is a stock
     torch.optim.SGD / Adam / AdamW and no GradScaler is active, its n per-particle steps
     (svgd.py:92-103) run inside the apply kernel (fused_base.py); set it to False to always call
-    `base_optimizer.step()` per particle.
+    `base_optimizer.step()` per particle.  Above 32 particles (ops.FUSED_MAX_PARTICLES) the fused form does not
+    exist: K2 writes the new gradients and the base optimizer steps per particle whatever this attribute says.
 
     `reuse_pair_distances` (class attribute, default True): the fused launch also computes the pair
     distances of the particles it has just updated (n <= 10), which are exactly what `rbf` needs at the
@@ -64,6 +71,8 @@ class SVGDOptimizer(BayesianOptimizer):
 
     def __init__(self, params, reset_params_closure, base_optimizer, particle_count, dataset_size, l2_reg=0.0,
                  kernel_grad_scale=1.0, process_group=None):
+        if particle_count > ops.MAX_PARTICLES:
+            raise ValueError(f"SVGDOptimizer supports at most {ops.MAX_PARTICLES} particles, got {particle_count}")
         params = list(params)
         super().__init__(map(lambda p: {"params": p}, params), {})
         self.state["__base_optimizer"] = base_optimizer
@@ -214,7 +223,8 @@ class SVGDOptimizer(BayesianOptimizer):
         return self._out_full
 
     def _plan_for(self, base, grad_scaler, plist):
-        if not self.fuse_base_optimizer or (grad_scaler is not None and grad_scaler.is_enabled()):
+        if (not self.fuse_base_optimizer or (grad_scaler is not None and grad_scaler.is_enabled())
+                or self.state["__particle_count"] > ops.FUSED_MAX_PARTICLES):
             return None
         plan = self._fused_plan
         if plan is None or plan.base is not base or not plan.still_valid():

@@ -37,7 +37,17 @@ extern "C" {
 #define BDE_ERR_WORKSPACE (-3)
 #define BDE_ERR_UNSUPPORTED_N (-4)
 
-#define BDE_MAX_PARTICLES 32
+/*
+ * Particle counts: every SVGD entry accepts 1 <= n <= BDE_MAX_PARTICLES (BDE_ERR_INVALID_ARG otherwise).
+ *   n <= 32: every SVGD entry, any alignment.
+ *   33 <= n <= 64: bde_svgd_workspace_bytes, bde_svgd_pairdist, bde_svgd_bandwidth, bde_svgd_pairdist_bandwidth,
+ *     bde_svgd_apply and bde_svgd_step only, on 16-byte aligned base pointers with ld % 4 == 0 (BDE_ERR_ALIGNMENT
+ *     otherwise); the fused base-optimizer entries (bde_svgd_apply_sgd / _adam, bde_svgd_train_step_*) and the
+ *     host-buffer entries (bde_svgd_host_*, bde_svgd_step_host) return BDE_ERR_UNSUPPORTED_N, and so does K1 on a
+ *     workspace attached to a peer set (bde_peer_attach; the exchange carries at most 32*31/2 sums): D-sharded jobs
+ *     all-reduce `dist` between bde_svgd_pairdist and bde_svgd_bandwidth instead.
+ */
+#define BDE_MAX_PARTICLES 64
 
 typedef void* bde_stream_t;
 
@@ -354,7 +364,7 @@ int bde_prior_terms_value_and_grad(int count, const int32_t* kinds_host, const u
  * sums with NaN after the attach-time timeout instead of hanging the GPU (bde_peer_status and the host status word
  * report it).
  *
- * Protocol (the library keeps no state; the caller owns everything):
+ * Protocol (the caller owns everything; the library only remembers which workspaces are attached):
  *   1. each rank: bde_peer_alloc -> device buffer + a BDE_PEER_HANDLE_BYTES CUDA-IPC handle;
  *   2. exchange the handles between the ranks (any host transport, e.g. torch.distributed);
  *   3. each rank: bde_peer_open on every OTHER rank's handle -> mapped device pointers;
