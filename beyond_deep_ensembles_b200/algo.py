@@ -44,7 +44,12 @@ class BayesianOptimizer(Optimizer):
 
     def load_state_dict(self, state_dict):
         from . import noise
+        base = self.state.get("__base_optimizer")
         super().load_state_dict(state_dict)
+        if base is not None and self.state.get("__base_optimizer", base) is None:
+            # a full state dict of a D-sharded job (ColumnShardedModel.full_state_dict) carries no base optimizer
+            # object (its state is a dict of its own): keep this optimizer's
+            self.state["__base_optimizer"] = base
         noise.restore_stream_position(state_dict.get("bde_noise_stream"))
 
     # ---- what subclasses implement (algo.py:19-56) ----

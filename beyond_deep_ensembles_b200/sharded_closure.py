@@ -25,16 +25,24 @@ With rank r's Philox counters starting at r * shard (dist.column_shard's prefix 
 closure equals the unsharded run on the same layout: bit for bit for the elementwise family when the ranks see
 the same batch, to rounding for SVGD (the n x n distance sums are added in a different order).
 
+Checkpoints: `full_state_dict(optimizer)` / `load_full_state_dict(optimizer, state_dict)` convert between a D-sharded
+optimizer's (or its base optimizer's) rank slices and the state dict of the same class constructed unsharded over the
+model's own parameters (checkpoint.py), so a job saved at R ranks resumes at any other R, and the plain classes (or
+the reference's) load and evaluate its checkpoint on one GPU.
+
 Not covered: an active GradScaler (each rank would run the non-finite check on its own columns only and the ranks
 could disagree about skipping a step; the D-sharded optimizers raise in step()), BBB / Rank-1 layers (their variational parameters live inside the modules and the layers sample in
-`forward`; `BBBOptimizer(process_group=...)` shards them per tensor), module buffers (rank-local, as under DDP
-without buffer broadcast), non-fp32 parameters.
+`forward`; `BBBOptimizer(process_group=...)` shards them per tensor and has no full state dict), D-sharded optimizers
+over slices made without this class (their global shapes are unknown to it), module buffers (rank-local, as under DDP
+without buffer broadcast, and not part of the optimizer state dicts), `torch.distributed.checkpoint` formats,
+non-fp32 parameters.
 """
 from __future__ import annotations
 
 import torch
 import torch.distributed as dist
 
+from . import checkpoint
 from . import dist as bdist
 from .layout import ALIGN, ParamLayout
 
@@ -191,3 +199,27 @@ class ColumnShardedModel:
         parts = [torch.empty_like(rows) for _ in range(self.world)]
         dist.all_gather(parts, rows, group=self._pg())
         return torch.cat(parts, dim=1)
+
+    # ------------------------------------------------------------------ checkpoints
+    def full_state_dict(self, optimizer) -> dict:
+        """The state dict `optimizer`'s class returns when constructed UNSHARDED over the model's own parameters
+        (`model.parameters()`, same order) after the same steps: same keys, per-parameter indices, shapes, dtypes and
+        devices, and `bde_noise_stream` (the furthest rank's).  `optimizer`: a SVGDOptimizer / SwagOptimizer /
+        iVONOptimizer over `[self.param]` with this group, or the torch.optim base optimizer over `[self.param]`.
+        `__base_optimizer` is None: save `full_state_dict(base)` beside it.
+
+        Collective over the group (one all_gather_object, one all_gather); every rank gets the same dict.  Memory:
+        what the unsharded optimizer holds — every column vector at full length D on `param`'s device on EVERY rank
+        (SVGD: n particles x D, iVON: 5 x D), SWAG's mean, second moment and [D, K] deviations on the host — plus one
+        [rows, R * shard] gather buffer on the device while it runs."""
+        return checkpoint.full_state_dict(self, optimizer)
+
+    def load_full_state_dict(self, optimizer, state_dict: dict) -> None:
+        """The inverse of `full_state_dict`: this rank's columns [lo, hi) of every vector, handed to the optimizer's own
+        `load_state_dict`.  Accepts a dict written by `full_state_dict` at any rank count, or by the plain class over
+        the model's parameters (this package's or the reference's).  The optimizer keeps its own base optimizer; load
+        the base optimizer's dict into it the same way.  No collective.
+
+        Raises ValueError — before anything is written — for another logical size or parameter shape, an optimizer
+        not over `[self.param]`, another `particle_count` / `deviation_samples`, or BBBOptimizer."""
+        checkpoint.load_full_state_dict(self, optimizer, state_dict)
