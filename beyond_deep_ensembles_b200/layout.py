@@ -35,6 +35,11 @@ class ParamLayout:
         self._index = {}
         self._copy_table = None
 
+    @classmethod
+    def from_shapes(cls, shapes, align: int = ALIGN) -> "ParamLayout":
+        """The layout of parameters of these shapes (it depends on nothing else): meta tensors, no storage."""
+        return cls([torch.empty(s, device="meta") for s in shapes], align)
+
     @property
     def copy_table(self):
         """The constant argument tables of ops.multi_tensor_copy for this layout (built on first use)."""

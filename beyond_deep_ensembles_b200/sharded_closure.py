@@ -25,14 +25,17 @@ With rank r's Philox counters starting at r * shard (dist.column_shard's prefix 
 closure equals the unsharded run on the same layout: bit for bit for the elementwise family when the ranks see
 the same batch, to rounding for SVGD (the n x n distance sums are added in a different order).
 
-Checkpoints: `full_state_dict(optimizer)` / `load_full_state_dict(optimizer, state_dict)` convert between a D-sharded
-optimizer's (or its base optimizer's) rank slices and the state dict of the same class constructed unsharded over the
-model's own parameters (checkpoint.py), so a job saved at R ranks resumes at any other R, and the plain classes (or
-the reference's) load and evaluate its checkpoint on one GPU.
+Checkpoints (checkpoint.py), two routes; a job saved at R ranks resumes at any other R by either.
+`full_state_dict(optimizer)` / `load_full_state_dict(optimizer, state_dict)` convert between a D-sharded optimizer's (or
+its base optimizer's) rank slices and the state dict of the same class constructed unsharded over the model's own
+parameters, so the plain classes (or the reference's) load and evaluate its checkpoint on one GPU; it puts the whole
+unsharded state on every rank.  `shard_state_dict(optimizer)` returns this rank's columns only, on the host, for each
+rank to save on its own; `load_shard_state_dicts(optimizer, shards)` reshards the R saved dicts by range arithmetic,
+and `checkpoint.consolidate(shards)` turns them into the full dict in one process.  Neither issues a collective.
 
 Not covered: an active GradScaler (each rank would run the non-finite check on its own columns only and the ranks
 could disagree about skipping a step; the D-sharded optimizers raise in step()), BBB / Rank-1 layers (their variational parameters live inside the modules and the layers sample in
-`forward`; `BBBOptimizer(process_group=...)` shards them per tensor and has no full state dict), D-sharded optimizers
+`forward`; `BBBOptimizer(process_group=...)` shards them per tensor and has neither checkpoint route), D-sharded optimizers
 over slices made without this class (their global shapes are unknown to it), module buffers (rank-local, as under DDP
 without buffer broadcast, and not part of the optimizer state dicts), `torch.distributed.checkpoint` formats,
 non-fp32 parameters.
@@ -53,6 +56,12 @@ class ColumnShardedModel:
     `model`: an nn.Module or an iterable of parameters (those with requires_grad are sharded).  Collective over the
     group at construction (rank 0's initial weights are broadcast unless `broadcast_init=False`).
     `average_grads`: reduce-scatter with AVG (data-parallel mean, default) or SUM.
+
+    Checkpoints: `full_state_dict` / `load_full_state_dict` (the reference-layout dict, gathered on every rank: for
+    evaluation on one GPU and for jobs whose whole state fits one rank twice) and `shard_state_dict` /
+    `load_shard_state_dicts` (each rank saves its own columns, the loader reshards to any rank count; no collective,
+    no length-D buffer).  Not covered by either: BBB / Rank-1 layers, module buffers, `torch.distributed.checkpoint`
+    formats.
     """
 
     def __init__(self, model, process_group=None, average_grads: bool = True, broadcast_init: bool = True):
@@ -223,3 +232,22 @@ class ColumnShardedModel:
         Raises ValueError — before anything is written — for another logical size or parameter shape, an optimizer
         not over `[self.param]`, another `particle_count` / `deviation_samples`, or BBBOptimizer."""
         checkpoint.load_full_state_dict(self, optimizer, state_dict)
+
+    def shard_state_dict(self, optimizer) -> dict:
+        """This rank's part of a per-rank checkpoint: a plain, picklable dict of `optimizer`'s rank-local state dict
+        (every tensor copied to the host, `__base_optimizer` None) and the column geometry — `format`, `version`,
+        `kind` (the optimizer's class name), `world`, `rank`, `shard`, `lo`, `hi` and the model's parameter `shapes`.
+        Nothing in it has length D.  `optimizer`: as for `full_state_dict`.  No collective: each rank
+        `torch.save`s its own dict.  Memory: one host copy of the rank-local state."""
+        return checkpoint.shard_state_dict(self, optimizer)
+
+    def load_shard_state_dicts(self, optimizer, shards) -> None:
+        """Load the R dicts `shard_state_dict` returned on the ranks of a saving job (any order, any R, typically
+        `torch.load(..., mmap=True)`): this rank's columns are cut from the saved shards that overlap [lo, hi), padding
+        columns keep the optimizer's values, and the rank-local dict goes to the optimizer's own `load_state_dict` —
+        the same dict `load_full_state_dict` builds from the full dict of that job.  No collective.
+
+        Raises ValueError — before anything is written — for dicts of another format, shards that do not tile the
+        saving job's columns exactly once, another logical size or parameter shape, another optimizer class, another
+        `particle_count` / `deviation_samples`, shards that disagree about a scalar, or BBBOptimizer."""
+        checkpoint.load_shard_state_dicts(self, optimizer, shards)
