@@ -452,15 +452,20 @@ svgd_pairdist_kernel(const float* __restrict__ X, int64_t D, int64_t ld, double*
 // ---------------------------------------------------------------------------------
 // K1, TMA-staged: one persistent CTA per SM; a producer warp streams [N x TC]-column tiles of X
 // into a shared-memory ring with cp.async.bulk, consumer warps accumulate the pair distances of
-// one column quad per thread per tile.  Besides keeping ~200 KB per SM in flight, this leaves
+// one column quad per thread per tile.  Besides keeping a ring of tiles per SM in flight, this leaves
 // only gridDim = #SMs partial sets for the deterministic last-CTA reduction.
 // ---------------------------------------------------------------------------------
 __host__ __device__ constexpr int pd_tile_cols(int n) {
     return pair_groups(n) == 1 ? 1024 : (pair_groups(n) == 2 ? 512 : (pair_groups(n) <= 4 ? 256 : 128));
 }
 __host__ __device__ constexpr int pd_stage_bytes(int n) { return n * pd_tile_cols(n) * 4; }
+// Ring size.  One pair group (n <= 10, 1024-column tiles): ~120 KB.  The read-only stream of [10 x 1024] tiles runs at
+// 7.3 TB/s through 3 stages, 7.1 through 4, 6.9 through 5 or 2, whichever way the copies are issued
+// (tools/microbench/stream_mix.cu, profiles/r03_stream_mix.jsonl); K1 itself is 4-8 % faster than with the ~200 KB
+// ring at n = 5, 8, 10.  At n = 12 a 120 KB ring is 3.5 % slower, so n >= 11 keeps ~200 KB (profiles/r03_ab_k1.jsonl).
+__host__ __device__ constexpr int pd_ring_bytes(int n) { return (pair_groups(n) == 1 ? 120 : 200) * 1024; }
 __host__ __device__ constexpr int pd_stages(int n) {
-    return (200 * 1024) / pd_stage_bytes(n) > 8 ? 8 : (200 * 1024) / pd_stage_bytes(n);
+    return pd_ring_bytes(n) / pd_stage_bytes(n) > 8 ? 8 : pd_ring_bytes(n) / pd_stage_bytes(n);
 }
 // consumer threads: one column quad of the tile per thread and pair group (256; 192 at n = 16)
 __host__ __device__ constexpr int pd_consumers(int n) { return pair_groups(n) * pd_tile_cols(n) / 4; }
@@ -1281,12 +1286,14 @@ int launch_apply_tma(const float* X, const float* G, float* out, const float* K,
     if (rc == BDE_OK) rc = encode_rows_tensor_map(&mapG, G, N, d4, ldg, kTmaBoxCols);
     if (rc != BDE_OK) return rc;
     int nst = apply_stages(N, OPT, TC);
-    // Ring depth in use.  With tensor-map loads the producer is no longer the limit, and for the plain K2 at n <= 12 a
-    // ~128 KB ring streams faster than the whole ~164-200 KB one (interleaved same-build A/B, profiles/r02_ring_ab.jsonl:
-    // n = 10 -5.6 %, n = 5 -1.4 %, n = 8 +-0; n = 16 / 20 and the fused forms are best or mixed at full depth) — fewer
-    // reads in flight leave the DRAM queues room for the write stream.  bde_tune("ring_kb") overrides (A/B runs).
+    // Ring depth in use.  With tensor-map loads the producer is no longer the limit, and the plain K2 at n <= 12 streams
+    // faster through a shallower ring than the whole ~164-200 KB one — fewer reads in flight leave the DRAM queues room
+    // for the write stream.  Interleaved same-build A/B against 128 KB (profiles/r03_ab_ring.jsonl): 100 KB is 4-7 %
+    // faster at n = 5, 8, 10 and 5 % slower at n = 12, which keeps 128 KB (profiles/r02_ring_ab.jsonl: 128 KB against the
+    // whole ring, n = 10 -5.6 %; n = 16 / 20 and the fused forms are best or mixed at full depth).  bde_tune("ring_kb")
+    // overrides (A/B runs).
     int ring_kb = tuning().ring_kb;
-    if (ring_kb == 0 && OPT == kOptNone && !NEXT && N <= 12) ring_kb = 128;
+    if (ring_kb == 0 && OPT == kOptNone && !NEXT && N <= 12) ring_kb = N <= 10 ? 100 : 128;
     if (ring_kb > 0) {
         const int want = ring_kb * 1024 / apply_stage_bytes(N, OPT, TC);
         if (want < nst) nst = want > TS + 1 ? want : TS + 1;
