@@ -88,12 +88,39 @@ class BayesianOptimizer(Optimizer):
             key = id(optimizer if optimizer is not None else self)
             grad_scaler._per_optimizer_states[key]["stage"] = stage
 
-    def _refuse_scaler_if_sharded(self, grad_scaler, world: int) -> None:
-        """D-sharded optimizers (process_group=...) see one rank's columns only: the non-finite check of an active
-        GradScaler would be taken per rank and the ranks could disagree about skipping a step — refuse loudly."""
-        if world > 1 and _scaler_active(grad_scaler):
-            raise ValueError("a D-sharded optimizer (process_group=...) does not support an active GradScaler: the "
-                             "non-finite check would have to be agreed over the group")
+    def _refuse_scaler_if_sharded(self, grad_scaler, world: int, group=None) -> None:
+        """D-sharded optimizers (process_group=`group`) see one rank's columns only, so the non-finite check of an
+        active GradScaler must be agreed over the group, or the ranks could disagree about skipping a step and back
+        the loss scale off differently.  torch's ShardedGradScaler over the same ranks agrees: its unscale_
+        all-reduces found_inf over its process group, and the fused gather route agrees on its flag in
+        `_agree_on_found_inf`.  Any other active scaler (a plain GradScaler, a look-alike, a ShardedGradScaler over
+        other ranks) is refused loudly."""
+        if world <= 1 or not _scaler_active(grad_scaler):
+            return
+        from torch.distributed.fsdp.sharded_grad_scaler import ShardedGradScaler
+        from . import dist as bdist
+        if not (isinstance(grad_scaler, ShardedGradScaler) and bdist.same_ranks(grad_scaler.process_group, group)):
+            raise ValueError("a D-sharded optimizer (process_group=...) supports an active GradScaler only as a "
+                             "torch.distributed.fsdp.sharded_grad_scaler.ShardedGradScaler over the same ranks: the "
+                             "non-finite check has to be agreed over the group")
+
+    def _agree_on_found_inf(self, grad_scaler, world: int, optimizer=None) -> None:
+        """D-sharded, fused route: MAX over the group of the non-finite flag the gathers of this step left in the
+        scaler's record for `optimizer` (default: self), so every rank's grad_scaler.step() / update() decide as the
+        unsharded job does.  The reference route needs nothing here (ShardedGradScaler.unscale_ agrees itself).
+
+        Called ONCE per step, after the last gather, not once per gather.  Every gather writes a fresh flag into the
+        record, as unscale_ does, and nothing reads it before the next gather replaces it: `_unscale_and_gather`
+        returns the literal algo.py:73 check, which reads the optimizer's own state, never the scaler's.  What the
+        scaler decides on (SVGD's grad_scaler.step(base) per particle, then update()) is the record after the
+        last gather of the step, and the MAX of that flag over the ranks is exactly the unsharded flag.  iVON needs
+        the agreement after its last parameter group, too: `_gather_more` raises the same flag."""
+        if world <= 1 or not (_scaler_active(grad_scaler) and self.fuse_unscale_into_gather):
+            return
+        from . import dist as bdist
+        record = grad_scaler._per_optimizer_states[id(self if optimizer is None else optimizer)]
+        for flag in record["found_inf_per_device"].values():
+            bdist.allreduce_max_(flag, grad_scaler.process_group)
 
     #: with an active GradScaler, fold unscale_ + the non-finite check into the gradient gather (SURVEY §8 f2)
     fuse_unscale_into_gather = True

@@ -108,7 +108,8 @@ class BBBOptimizer(BayesianOptimizer):
 
     def step(self, forward_closure, backward_closure, grad_scaler=None):
         if grad_scaler is not None:
-            self._refuse_scaler_if_sharded(grad_scaler, bdist.world(self._group))
+            # grad_scaler.step(base) runs the scaler's own unscale_, which a ShardedGradScaler agrees over the group
+            self._refuse_scaler_if_sharded(grad_scaler, bdist.world(self._group), self._group)
         base = self.state["__base_optimizer"]
         base.zero_grad()
 

@@ -112,6 +112,24 @@ def allreduce_scalar_value(value: torch.Tensor, group) -> torch.Tensor:
     return value + (total - value.detach())
 
 
+def same_ranks(a, b) -> bool:
+    """True when groups `a` and `b` hold the same global ranks (None = the default group).  False for a group this
+    rank is not a member of (torch.distributed.new_group hands non-members a placeholder)."""
+    if a is b:
+        return True
+    try:
+        return sorted(dist.get_process_group_ranks(a)) == sorted(dist.get_process_group_ranks(b))
+    except (KeyError, RuntimeError, ValueError):
+        return False
+
+
+def allreduce_max_(flag: torch.Tensor, group) -> torch.Tensor:
+    """In place: the largest value of a device scalar over the ranks holding the other column slices (the non-finite
+    flag of a gradient gather).  Enqueued on the stream like any collective; no host synchronisation."""
+    dist.all_reduce(flag, op=dist.ReduceOp.MAX, group=group)
+    return flag
+
+
 # --------------------------------------------------------------------------------------
 # in-kernel exchange over peer memory
 # --------------------------------------------------------------------------------------

@@ -75,7 +75,8 @@ class iVONOptimizer(BayesianOptimizer):
 
     # ------------------------------------------------------------------ step
     def step(self, forward_closure, backward_closure, grad_scaler=None):
-        self._refuse_scaler_if_sharded(grad_scaler, self._arenas[0]["shard"].world)
+        shard = self._arenas[0]["shard"]
+        self._refuse_scaler_if_sharded(grad_scaler, shard.world, shard.group)
         self._reset_state()
         self._drop_presampled(release=True)   # training does not keep the prediction-time sample buffers
 
@@ -118,6 +119,7 @@ class iVONOptimizer(BayesianOptimizer):
             # arena holds the sum so far (zeros before the first sample), so the ordinary path continues from it
             if not self._store_gradients(grad_scaler):   # unscale (if AMP) + gather-accumulate, one launch per group
                 return None
+        self._agree_on_found_inf(grad_scaler, shard.world)   # D-sharded: the last sample's flag, all groups raised
         acc_loss /= self.mc_samples
 
         with torch.no_grad():

@@ -33,8 +33,12 @@ unsharded state on every rank.  `shard_state_dict(optimizer)` returns this rank'
 rank to save on its own; `load_shard_state_dicts(optimizer, shards)` reshards the R saved dicts by range arithmetic,
 and `checkpoint.consolidate(shards)` turns them into the full dict in one process.  Neither issues a collective.
 
-Not covered: an active GradScaler (each rank would run the non-finite check on its own columns only and the ranks
-could disagree about skipping a step; the D-sharded optimizers raise in step()), BBB / Rank-1 layers (their variational parameters live inside the modules and the layers sample in
+Mixed precision: each rank checks only its own columns for non-finite gradients, so the D-sharded optimizers accept an
+active scaler only as torch's `ShardedGradScaler` over the optimizer's ranks. The ranks then agree on every skipped step
+and on the loss scale. Anything else raises in step(). The scaler's `state_dict()` is the same on every rank: a
+checkpoint saves it once beside the optimizer's dicts.
+
+Not covered: BBB / Rank-1 layers (their variational parameters live inside the modules and the layers sample in
 `forward`; `BBBOptimizer(process_group=...)` shards them per tensor and has neither checkpoint route), D-sharded optimizers
 over slices made without this class (their global shapes are unknown to it), module buffers (rank-local, as under DDP
 without buffer broadcast, and not part of the optimizer state dicts), `torch.distributed.checkpoint` formats,

@@ -128,8 +128,9 @@ class SVGDOptimizer(BayesianOptimizer):
         losses = []
         prebind = self._prebind_active(grad_scaler, self._layout.size, len(plist))
         scaler_on = grad_scaler is not None and grad_scaler.is_enabled()
+        world = bdist.world(self._group)
         if scaler_on:
-            self._refuse_scaler_if_sharded(grad_scaler, bdist.world(self._group))
+            self._refuse_scaler_if_sharded(grad_scaler, world, self._group)
         if prebind:
             self._G.zero_()   # ONE memset for all particles; autograd then accumulates straight into the arena rows
         for particle_idx in range(n):
@@ -160,6 +161,8 @@ class SVGDOptimizer(BayesianOptimizer):
             # gather: the closure replaced a .grad (zero_grad(set_to_none=True) inside it), AMP, or prebinding off
             if not self._store_grads(particle_idx, plist, grad_scaler, base):   # unscale (if AMP) + gather, one launch
                 return None
+        if scaler_on:
+            self._agree_on_found_inf(grad_scaler, world, base)   # D-sharded: the last particle's flag decides
         # mean over the particles (svgd.py:105) in ONE reduction instead of n accumulate launches
         mean_loss = torch.stack(losses).mean() if n > 1 else losses[0].clone()
 

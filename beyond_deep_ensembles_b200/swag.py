@@ -73,7 +73,8 @@ class SwagOptimizer(BayesianOptimizer):
 
     # ------------------------------------------------------------------ step
     def step(self, forward_closure, backward_closure, grad_scaler=None):
-        self._refuse_scaler_if_sharded(grad_scaler, self._shard.world)
+        # no gather on this path: grad_scaler.step(base) runs the scaler's own unscale_, which a ShardedGradScaler agrees
+        self._refuse_scaler_if_sharded(grad_scaler, self._shard.world, self._shard.group)
         self._drop_presampled(release=True)   # the posterior is about to change; training does not keep the buffer
         self._restore_original_params()
         base = self.state["__base_optimizer"]
